@@ -28,6 +28,10 @@ partition set instead.  Q6 over SF-10 is measured in the same run and reported u
 `parity_check`: in the same run the oracle's generated-loop layer (CPU) scans the SAME ColumnBatch bytes at the
 benchmark's own size (every rank its shard; partial rows gathered and merged) and the GPU result must match: counts
 bit-exact, DOUBLE sums / averages within 1e-6 relative (BASELINE.json north_star).  A mismatch fails the run.
+
+`--dump-outputs DIR` writes the final rows of the last timed step of Q1 and Q6 as .npy files.  The tables are generated
+on the device from fixed seeds, so the same arguments give the same inputs on every run and two builds can be compared
+output for output.
 """
 import argparse
 import ctypes as C
@@ -70,7 +74,34 @@ def parse_args():
                     help="N > 1: strong (default, BASELINE.json: ONE SF-100 table over 1->8 GPUs) = the table split into N contiguous "
                          "batch ranges, one partition set per GPU; weak = every rank scans its own table-sized partition set")
     ap.add_argument("--no-parity", action="store_true", help="skip the GPU-vs-oracle parity check at the benchmark's own size")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the final rows of the last timed step of each Q1 / Q6 query to DIR/<query>_keys.npy and "
+                         "DIR/<query>_values.npy (float64), so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "native" or args.workload not in ("q1", "q6")):
+        ap.error("--dump-outputs covers the Q1 / Q6 queries of the native implementation")
+    return args
+
+
+def dump_final_rows(out_dir, name, rows, desc):
+    """Final rows of one query as float64 arrays, groups sorted by key: <name>_keys.npy (groups, keys, longest key) holds
+    the bytes of the string keys, zero-padded (Q6 has no keys and no such file); <name>_values.npy (groups, aggregates)
+    the aggregates, NULL as NaN."""
+    import numpy as np
+    nkeys = len(desc.keys_py)
+    rows = sorted(rows, key=lambda r: tuple(r[:nkeys]))
+    os.makedirs(out_dir, exist_ok=True)
+    if nkeys:
+        width = max((len(k) for r in rows for k in r[:nkeys]), default=0)
+        keys = np.zeros((len(rows), nkeys, width), dtype=np.float64)
+        for i, r in enumerate(rows):
+            for j, k in enumerate(r[:nkeys]):
+                keys[i, j, :len(k)] = np.frombuffer(k, dtype=np.uint8)
+        np.save(os.path.join(out_dir, name + "_keys.npy"), keys)
+    values = np.array([[np.nan if v is None else float(v) for v in r[nkeys:]] for r in rows], dtype=np.float64)
+    np.save(os.path.join(out_dir, name + "_values.npy"), values.reshape(len(rows), len(desc.final_schema()) - nkeys))
 
 
 def ncu_traffic_per_row(q1):
@@ -660,6 +691,8 @@ def main():
     launches_timed = main_run.launches * args.steps // nsteps_all
     d2h_step = 0
     final_rows = capi.parse_row_stream(main_run.final_raw, main_run.desc.final_schema())
+    if args.dump_outputs and rank == 0:
+        dump_final_rows(args.dump_outputs, args.workload, final_rows, main_run.desc)
 
     out = {"metric": metric_name(q1), "value": job_rows * args.steps / (ms / 1e3), "unit": "rows/s", "n_gpus": world,
            "steps": args.steps, "warmup": args.warmup, "ms_per_step": ms / args.steps, "higher_is_better": True,
@@ -759,6 +792,9 @@ def main():
         ototal = SF100_ROWS if oq1 else SF10_ROWS
         other = QueryRun(api, torch, dist, oq1, ototal, rank, world, local_rank, args.scaling, comm)
         oms = timed_steps(torch, dist, world, other.step_resident, args.warmup, args.steps)
+        if args.dump_outputs and rank == 0:
+            dump_final_rows(args.dump_outputs, "q1" if oq1 else "q6",
+                            capi.parse_row_stream(other.final_raw, other.desc.final_schema()), other.desc)
         okms = other.kernel_ns / 1e6 / max(1, other.launches)
         oalgo = other.algo_bytes / max(1, other.launches)
         out["also"] = {"workload": workload_config(oq1, ototal, world, args.scaling)["workload"], "value": other.job_rows * args.steps / (oms / 1e3),

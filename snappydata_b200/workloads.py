@@ -72,7 +72,6 @@ def c4_base_batch(k: int):
 
 def run_c4(api, torch, dist, rank, world, device, steps, warmup, peak):
     from oracle import oracle
-    steps = max(1, min(steps, 5))
     first_row, nrows, nb = shard_batches(C4_TOTAL_ROWS, ROWS_PER_BATCH, rank, world)
     b0 = first_row // ROWS_PER_BATCH
     need = sorted({(b0 + i) % C4_BASE_BATCHES for i in range(nb)})
@@ -163,7 +162,6 @@ def _decorate_hybrid(cb: ColumnBatch, r):
 def run_c5(api, torch, device, steps, warmup, peak, total_rows=59_986_052, ingest_batches=60):
     """1 GPU.  -> JSON-able dict with value (rows/s over the snapshots actually scanned), roofline and the parity assertion."""
     from oracle import oracle
-    steps = max(1, min(steps, 40))
     r = np.random.default_rng(5)
     desc = P.q6_plan()
     cols = desc.table_cols

@@ -1,6 +1,6 @@
 """Runs bench.py's main() with the GPU, the C-ABI library and torch.distributed replaced by stand-ins, so that the
 host-side logic of the bench (sharding modes, per-job row accounting, the JSON line) is exercised without a GPU.
-usage: python bench_mock.py WORLD weak|strong   (driven by tests/test_bench_line.py)"""
+usage: python bench_mock.py WORLD weak|strong [bench.py arguments]   (driven by tests/test_bench_line.py)"""
 import sys, types, importlib.util, ctypes as C, json
 ROOT = __import__('os').path.dirname(__import__('os').path.dirname(__import__('os').path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -65,7 +65,7 @@ capi.Comm = FakeComm
 capi.product_api = lambda: FakeApi()
 capi.Store = FakeStore
 capi.Plan = FakePlan
-capi.parse_row_stream = lambda raw, schema: []
+capi.parse_row_stream = lambda raw, schema: [[b"N" if t == capi.SqlType.STRING else 1.0 for t in schema]]
 class FakeMB:
     def __init__(self, cb, cols):
         self.c = capi.sd_batch(); self.c.num_rows = cb.num_rows; self.c.batch_id = cb.batch_id; self.c.bucket_id = cb.bucket_id
@@ -96,7 +96,7 @@ class FakeEx:
 ex.PartialRowExchange = FakeEx
 _print = print
 
-sys.argv = ["bench.py", "--gpus", str(WORLD), "--scaling", SCALING, "--rows", "1000001", "--steps", "2", "--warmup", "1"]
+sys.argv = ["bench.py", "--gpus", str(WORLD), "--scaling", SCALING, "--rows", "1000001", "--steps", "2", "--warmup", "1"] + sys.argv[3:]
 b.main()   # last rank: prints nothing unless WORLD == 1
 os.environ['RANK'] = '0'; os.environ['LOCAL_RANK'] = '0'
 if WORLD > 1:

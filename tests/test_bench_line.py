@@ -10,8 +10,9 @@ import pytest
 HERE = os.path.dirname(os.path.abspath(__file__))
 
 
-def run(world, scaling):
-    out = subprocess.run([sys.executable, os.path.join(HERE, "bench_mock.py"), str(world), scaling], capture_output=True, text=True, timeout=300)
+def run(world, scaling, *bench_args):
+    out = subprocess.run([sys.executable, os.path.join(HERE, "bench_mock.py"), str(world), scaling, *bench_args], capture_output=True,
+                         text=True, timeout=300)
     assert out.returncode == 0, out.stderr[-2000:]
     lines = [l for l in out.stdout.splitlines() if l.startswith("{")]
     assert len(lines) == 1, out.stdout[-2000:]
@@ -39,3 +40,18 @@ def test_bench_line(world, scaling):
         assert e["rows_per_step"] == job
     else:   # (the stand-in all-reduce multiplies rank 0's count, whose shard may hold one batch more than the others)
         assert abs(e["rows_per_step"] - job) <= world * 200_000
+
+
+@pytest.mark.parametrize("world", [1, 2])
+def test_bench_dumps_the_last_timed_step(world, tmp_path):
+    """--dump-outputs writes the final rows of Q1 (2 string keys, 8 aggregates) and of Q6 (1 aggregate) as float64 arrays;
+    --steps is the number of timed steps."""
+    import numpy as np
+    d = run(world, "strong", "--steps", "7", "--dump-outputs", str(tmp_path))
+    assert d["steps"] == 7
+    assert sorted(os.listdir(tmp_path)) == ["q1_keys.npy", "q1_values.npy", "q6_values.npy"]
+    keys, values, q6 = (np.load(tmp_path / f) for f in ("q1_keys.npy", "q1_values.npy", "q6_values.npy"))
+    assert keys.dtype == values.dtype == q6.dtype == np.float64
+    assert keys.shape == (1, 2, 1) and (keys == ord("N")).all()
+    assert values.shape == (1, 8) and (values == 1.0).all()
+    assert q6.shape == (1, 1)
